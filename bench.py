@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - keyframe depth maps/s of the CVA-MVSNet hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision mixed16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision mixed16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -9,7 +9,9 @@ A "step" is one DrMvsnet window (7 views, 640x480, 3 stages, depth_num (48,32,8)
 BASELINE.json configs[1]) through the hot path.  `value` times K steps with the window already resident in HBM
 (CUDA events on the engine's stream, max over ranks); `e2e` times the same K steps through the public
 DrMvsnet.CallAsync -> GetResult call with host buffers (pinned H2D of the u8 images and D2H of the four output maps
-inside the timed region).  Multi-GPU: one process per GPU, independent windows per rank (weak scaling, no data-path
+inside the timed region).  --dump-outputs DIR writes the four maps the end-to-end leg returned for its last step
+(rank 0; the inputs are the same on every run) as DIR/<name>.npy, so that two builds can be compared output for output.
+Multi-GPU: one process per GPU, independent windows per rank (weak scaling, no data-path
 collective - SURVEY.md §8e); torch.distributed is only used for the barrier and the max-over-ranks reduction.
 `--impl reference` times the reference's own CPU path: its PyTorch model cannot travel to the GPU box, so the
 pinned CPU restatement (oracle/mvsnet_oracle.py, verified against the reference model and its shipped goldens) is
@@ -27,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
 
 WORKLOAD = "CVA-MVSNet 640x480, 7 views, 3-stage cascade (48/32/8), view aggregation (abl03), 1 window/step/GPU"
 WEIGHTS = "abl03_view_aggregation"
@@ -328,13 +331,19 @@ def main():
                          "the extra host threads and staging buffers cost more than the added overlap gives")
     ap.add_argument("--tc", type=int, default=-1, help="1/0: force the tcgen05 conv path on/off (default: engine default)")
     ap.add_argument("--opt", action="append", default=[], help="engine option key=int for A/B runs, e.g. --opt fork_fpn=0")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result maps of the last timed end-to-end step as DIR/<name>.npy (float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "mvsnet"):
+        ap.error("--dump-outputs applies to the mvsnet workload of --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     host_malloc = tune_host_malloc()
     if a.workload == "slab_tsdf":
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import bench_slab_tsdf
-        r = bench_slab_tsdf.main(["--frames", str(min(a.steps, 48)), "--warmup", str(a.warmup)])
+        r = bench_slab_tsdf.main(["--frames", str(a.steps), "--warmup", str(a.warmup)])
         if r is not None:
             print(json.dumps({"metric": "TSDF depth maps integrated + ray-cast per second (1024^3 voxels @ 1 cm, Z-slab partition)",
                               "value": r["frames_per_s"], "unit": "frames/s", "n_gpus": r["n_gpus"], "steps": r["frames"],
@@ -350,7 +359,7 @@ def main():
         if rank != 0:
             return 0
         win = load_window(0)
-        steps = max(1, min(a.steps, 6))
+        steps = a.steps
         kfs, ms = time_cpu(win, steps, min(a.warmup, 1))
         cores = win["cpu_threads"]
         print(json.dumps({
@@ -444,8 +453,10 @@ def main():
         torch.cuda.synchronize(local)
         ms = (time.perf_counter() - t0) * 1e3
         assert np.isfinite(r.depth_dense).all()
+        last[0] = r
         return ms
 
+    last = [None]                           # the result of the last step of the latest e2e leg
     hs_e2e = hs[:max(1, min(a.e2e_inflight, len(hs)))]
     pin_outs = [DrMvsnetOutput(win["H"], win["W"], pinned=True) for _ in hs_e2e]
     for _ in range(2):
@@ -458,6 +469,10 @@ def main():
         submit_pinned(h); h.GetResult(out=o)
     ms_e2e_serial = e2e_leg(hs_e2e[:1], submit_pinned, pin_outs[:1])
     ms_e2e = e2e_leg(hs_e2e, submit_pinned, pin_outs) if len(hs_e2e) > 1 else ms_e2e_serial
+    if a.dump_outputs and rank == 0:        # the headline e2e leg's last step, copied before the buffers are reused
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name in ("depth", "confidence", "depth_dense", "confidence_dense"):
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), np.array(getattr(last[0], name), np.float32))
     for h in hs_e2e:
         h.set_option("eager_d2h", 1)
     assert np.array_equal(pin_outs[0].depth_dense, out.depth_dense), "page-locked and pageable paths must return the same map"

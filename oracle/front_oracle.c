@@ -16,8 +16,8 @@
  * CoarseTracker.cpp:655-725) and compiles them, unmodified, against a stand-in Eigen (tests/cpp/eigen_stub) and the harness
  * oracle/ref_wrap_front.cpp into oracle/_ref/libfront_ref.so; tests/test_oracle_cpu.py::test_front_oracle_*_pinned_* compare
  * this restatement with that library bit for bit (pyramid incl. a non-finite pixel; pc_n and all four point arrays for
- * steps 1-3, with and without sparse points, up to 640x480).  Without /root/reference (fresh clone) those tests skip and
- * the oracle is "parity unpinned".  Deliberate, documented deviations:
+ * steps 1-3, with and without sparse points, up to 640x480); what that library returned is stored in
+ * tests/golden/ref_front.npz (oracle/ref_golden.py), so the tests run without the reference.  Deliberate, documented deviations:
  *   * rows 0 and h-1 of (dx, dy, absSquaredGrad) are uninitialised memory in the reference (`new Eigen::Vector3f[]`);
  *     here they are 0.  The tracker never reads them (2 < Kv < h-3).
  *   * a warped depth <= 0 (point behind the reference camera) is ignored; in the reference its effect depends on the

@@ -9,7 +9,8 @@ unmodified, against a stand-in Eigen / SE3 (tests/cpp/eigen_stub, oracle/ref_wra
 tests/test_oracle_cpu.py::test_lm_driver_pinned_to_reference_trackNewestCoarse drives that loop and this restatement with the
 SAME tracker object and requires the same number of evaluations (= the same accept / reject sequence, cutoff doublings, stop
 iteration and level repeat) and the same pose / affine parameters, for free, fixed-a, fixed-b and fixed-a-b optimisation and
-a saturating start.  Without /root/reference the test skips and this file is "parity unpinned".  The restatement follows
+a saturating start; what that loop returned is stored in tests/golden/ref_lm.npz (oracle/ref_golden.py), so the test runs
+without the reference.  The restatement follows
 the listed lines statement by statement: cutoff doubling while the saturated ratio exceeds 0.6
 (:779-790), lambda = 0.01 (:798), H diagonal *(1+lambda) and LDLT solve on the free parameters (:814-840), the
 extrapolation factor (:843-845), SCALE_* (:847-851, cuda_coarse_tracker.cpp:12-19), left-multiplicative SE3 update

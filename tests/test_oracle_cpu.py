@@ -7,6 +7,8 @@ import torch
 
 from oracle import mvsnet_oracle as O
 from oracle.cpu import TrackerOracle, TsdfOracle
+from oracle.ref_golden import (FRONT_DENSE_CASES, FRONT_PYRAMID_CASES, LM_CASES, assert_exact, front_dense_case,
+                               front_pyramid_case, golden_path, lm_case, lm_key, lm_start, mvsnet_fresh_case)
 from tandem_b200 import DrFusionOptions, default_weights
 from tandem_b200.synthetic import RoomScene, look_at_pose, tracker_case
 from tandem_b200.weights_io import load_tdmw
@@ -37,35 +39,21 @@ def test_mvsnet_oracle_matches_reference_abl03(golden_small):
         assert ed < 2e-5, (s, ed)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/cva_mvsnet"), reason="reference tree not present")
 def test_oracle_matches_reference_model_on_fresh_input():
-    """Build-container only: the restatement equals the imported reference model on a seeded synthetic window."""
-    import sys
-    import types
-    sys.path.insert(0, "/root/reference/cva_mvsnet")
-    pkg = types.ModuleType("models"); pkg.__path__ = ["/root/reference/cva_mvsnet/models"]; sys.modules["models"] = pkg
-    from models.cva_mvsnet import CvaMVSNet, StageTensor
-    ck = torch.load("/root/reference/cva_mvsnet/pretrained/ablation/abl03_view_aggregation.ckpt", map_location="cpu",
-                    weights_only=False)
-    net = CvaMVSNet(depth_num=ck["hparams"]["MODEL.DEPTH_NUM"], view_aggregation=True).eval()
-    net.load_state_dict({k[len("cva_mvsnet."):]: v for k, v in ck["state_dict"].items()})
-    torch.manual_seed(0)
-    V, H, W = 4, 64, 96
-    img = torch.rand(V, 3, H, W)
-    img = torch.nn.functional.avg_pool2d(img, 5, 1, 2)
-    K3 = torch.tensor([[100.0, 0, 47.5], [0, 100.0, 31.5], [0, 0, 1]])
-    Ks = [torch.cat([K3[:2] * s, K3[2:]]) for s in (0.25, 0.5, 1.0)]
-    c2w = torch.eye(4).repeat(V, 1, 1)
-    c2w[:, 0, 3] = torch.arange(V) * 0.05
+    """The restatement equals the reference model (its stored outputs, oracle/ref_golden.py) on a seeded synthetic window."""
+    img, Ks, c2w, dmin, dmax, disc = mvsnet_fresh_case()
+    g = np.load(golden_path("ref_mvsnet_fresh.npz"))
+    assert np.array_equal(img.reshape(-1)[::997].numpy(), g["input_probe"]), "the seeded input window changed"
     with torch.no_grad():
-        ref = net(img[None], StageTensor(*[k[None] for k in Ks]), c2w[None], torch.tensor([0.5]), torch.tensor([5.0]),
-                  torch.tensor([10.0]))
         w, dn, va = load_tdmw(default_weights("abl03_view_aggregation"))
-        ours = O.forward(w, dn, img, Ks, c2w, 0.5, 5.0, 10.0, va)
+        ours = O.forward(w, dn, img, Ks, c2w, dmin, dmax, disc, va)
     for s in range(3):
-        assert (ref[s].depth_dense[0] - ours[s]["depth_dense"]).abs().max() < 1e-4
-        assert (ref[s].depth[0] - ours[s]["depth"]).abs().max() < 1e-4
-        assert (ref[s].confidence[0] - ours[s]["confidence"]).abs().max() < 1e-4
+        dense = g[f"stage{s + 1}_depth_dense"]
+        zero = np.unpackbits(g[f"stage{s + 1}_depth_zero"], count=dense.size).reshape(dense.shape).astype(bool)
+        depth = np.where(zero, np.float32(0), dense)
+        assert np.abs(dense - ours[s]["depth_dense"].numpy()).max() < 1e-4
+        assert np.abs(depth - ours[s]["depth"].numpy()).max() < 1e-4
+        assert np.abs(g[f"stage{s + 1}_confidence"] - ours[s]["confidence"].numpy()).max() < 1e-4
 
 
 def test_tsdf_oracle_basic_properties():
@@ -142,63 +130,36 @@ def test_front_oracle_pyramid_and_dense_reference():
     assert n3 == 2 + interior - 2 and arrs3[0][0] == 7 and arrs3[0][1] == 9
 
 
-def _front_ref():
-    from oracle.cpu import FrontRef
-    if not FrontRef.available():
-        pytest.skip("oracle/_ref/libfront_ref.so not built (needs /root/reference: make -C oracle -f ref_build.mk)")
-    return FrontRef()
-
-
-@pytest.mark.parametrize("size,levels", [((480, 640), 4), ((96, 130), 2), ((60, 80), 3)])
+@pytest.mark.parametrize("size,levels", FRONT_PYRAMID_CASES)
 def test_front_oracle_pyramid_pinned_to_reference_makeImages(size, levels):
     """n2 pin: oracle/front_oracle.c == the reference's own FrameHessian::makeImages body (HessianBlocks.cpp:128-191,
-    compiled unmodified into oracle/_ref/libfront_ref.so), bit for bit, incl. a non-finite input pixel."""
+    compiled unmodified by oracle/ref_build.mk; its outputs are stored by oracle/ref_golden.py), bit for bit, incl. a
+    non-finite input pixel."""
     from oracle.cpu import FrontOracle
-    ref = _front_ref()
-    h, w = size
-    rng = np.random.default_rng(3)
-    gray = (rng.random((h, w)) * 255).astype(np.float32)
-    gray[5, 7] = np.inf
-    a = FrontOracle().make_images(gray, levels)
-    b = ref.make_images(gray, levels)
+    g = np.load(golden_path("ref_front.npz"))
+    a = FrontOracle().make_images(front_pyramid_case(size), levels)
     for lvl in range(levels):
-        assert np.array_equal(a[lvl][0], b[lvl][0], equal_nan=True), f"level {lvl} (I,dx,dy)"
-        assert np.array_equal(a[lvl][1], b[lvl][1], equal_nan=True), f"level {lvl} absSquaredGrad"
+        key = f"pyr/{size[0]}x{size[1]}/{lvl}"
+        assert_exact(g, key + "/dI", a[lvl][0], f"level {lvl} (I,dx,dy)")
+        assert_exact(g, key + "/absSquaredGrad", a[lvl][1], f"level {lvl} absSquaredGrad")
 
 
-@pytest.mark.parametrize("step,with_sparse,size", [(1, False, (240, 320)), (2, True, (240, 320)), (1, True, (120, 160)),
-                                                    (3, False, (480, 640))])
+@pytest.mark.parametrize("step,with_sparse,size", FRONT_DENSE_CASES)
 def test_front_oracle_dense_reference_pinned_to_reference_setCoarseTrackingRef(step, with_sparse, size):
     """n1 pin: forward warp + nearest-depth test + raster-order append (incl. the ++pc_n quirk) of oracle/front_oracle.c ==
-    the reference's own dense block of CoarseTracker::setCoarseTrackingRef (CoarseTracker.cpp:655-725), bit for bit: pc_n,
-    all four point arrays and the stale / uncounted slots."""
+    the reference's own dense block of CoarseTracker::setCoarseTrackingRef (CoarseTracker.cpp:655-725, outputs stored by
+    oracle/ref_golden.py), bit for bit: pc_n, all four point arrays and the stale / uncounted slots."""
     from oracle.cpu import FrontOracle
-    ref = _front_ref()
-    h, w = size
-    f = 160.0 * w / 320.0
-    K4 = (f, f, (w - 1) / 2.0, (h - 1) / 2.0)
-    scene = RoomScene()
-    pose_d = look_at_pose((0.3, 0.0, -0.2), (2.5, 0.2, 0.5))
-    pose_r = look_at_pose((0.34, 0.02, -0.17), (2.5, 0.25, 0.45))
-    _, depth = scene.render(pose_d, h, w, *K4, dropout=0.02, seed=1)
-    bgr_r, _ = scene.render(pose_r, h, w, *K4)
-    gray_r = bgr_r.astype(np.float32) @ np.array([0.114, 0.587, 0.299], np.float32)
-    rng = np.random.default_rng(5)
-    sparse, idepth0 = None, None
-    if with_sparse:
-        ns = 500
-        sparse = [rng.integers(3, w - 3, ns + 1).astype(np.float32), rng.integers(3, h - 3, ns + 1).astype(np.float32),
-                  rng.uniform(0.2, 2.0, ns + 1).astype(np.float32), rng.uniform(0, 255, ns + 1).astype(np.float32)]
-        idepth0 = np.zeros((h, w), np.float32)
-        idepth0[sparse[1][:ns].astype(int), sparse[0][:ns].astype(int)] = sparse[2][:ns]
-    n_ref, arrs_ref, T = ref.dense_reference(depth, pose_d, pose_r.astype(np.float64), K4, step, not with_sparse, sparse,
-                                             idepth0, gray_r)
+    g = np.load(golden_path("ref_front.npz"))
+    key = f"dense/{step}/{int(with_sparse)}/{size[0]}x{size[1]}"
+    depth, pose_d, pose_r, K4, sparse, idepth0, gray_r = front_dense_case(step, with_sparse, size)
+    n_ref, T = int(g[key + "/n"]), g[key + "/T"]
     # the transform the reference derives (SE3 inverse * SE3) is the one the oracle / the device path is handed
     assert np.allclose(T, np.linalg.inv(pose_r.astype(np.float64)) @ pose_d.astype(np.float64), atol=1e-12)
     n, arrs, _ = FrontOracle().dense_reference(depth, T, K4, step, not with_sparse, sparse, idepth0, gray_r)
     assert n == n_ref and n > 1000
-    for a, b, name in zip(arrs, arrs_ref, ("u", "v", "idepth", "color")):
-        assert np.array_equal(a, b), name
+    for a, name in zip(arrs, ("u", "v", "idepth", "color")):
+        assert_exact(g, f"{key}/{name}", a, name)
 
 
 def test_lm_driver_converges_with_oracle_tracker():
@@ -220,54 +181,20 @@ def test_lm_driver_converges_with_oracle_tracker():
     assert np.allclose(se3_exp(np.zeros(6)), np.eye(4))
 
 
-@pytest.mark.parametrize("start,fix_a,fix_b,cutoff", [("identity", False, False, 20.0), ("near", False, False, 20.0),
-                                                       ("identity", True, True, 20.0), ("identity", False, True, 20.0),
-                                                       ("identity", True, False, 20.0), ("identity", False, False, 0.8)])
+@pytest.mark.parametrize("start,fix_a,fix_b,cutoff", LM_CASES)
 def test_lm_driver_pinned_to_reference_trackNewestCoarse(start, fix_a, fix_b, cutoff):
-    """n3 pin: oracle/lm_driver.py == the reference's own level loop (CoarseTracker.cpp:750-916 compiled unmodified into
-    oracle/_ref/liblm_ref.so) when both drive the SAME tracker object: same number of residual / normal-equation evaluations
-    (i.e. same accept / reject sequence, cutoff doublings and stop iteration), same pose and affine parameters.  The last case
-    starts with a cutoff so small that > 60 % of the points saturate: the cutoff-doubling and REPEAT-LEVEL rules run."""
-    import ctypes
+    """n3 pin: oracle/lm_driver.py == the reference's own level loop (CoarseTracker.cpp:750-916 compiled unmodified by
+    oracle/ref_build.mk; oracle/ref_golden.py stores what it returned) when both drive the SAME tracker object: same number
+    of residual / normal-equation evaluations (i.e. same accept / reject sequence, cutoff doublings and stop iteration), same
+    pose and affine parameters.  The last case starts with a cutoff so small that > 60 % of the points saturate: the
+    cutoff-doubling and REPEAT-LEVEL rules run."""
     from oracle.lm_driver import track_level0
-    lib_path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "liblm_ref.so")
-    if not os.path.exists(lib_path):
-        pytest.skip("oracle/_ref/liblm_ref.so not built (needs /root/reference: make -C oracle -f ref_build.mk)")
-    l = ctypes.CDLL(lib_path)
-    c = tracker_case(H=120, W=160, fx=80.0, fy=80.0, cx=79.5, cy=59.5)
-    t = TrackerOracle(c["w"], c["h"])
-    t.setK(c["w"], c["h"], c["fx"], c["fy"], c["cx"], c["cy"])
-    t.setReference(c["n"], c["pc_u"], c["pc_v"], c["pc_idepth"], c["pc_color"], c["ref_exposure"], c["ref_aff"])
-    t.setNew(c["dInew"])
-    dp = ctypes.POINTER(ctypes.c_double)
-    RES = ctypes.CFUNCTYPE(None, ctypes.c_void_p, dp, ctypes.c_float, dp, ctypes.c_float, dp)
-    G = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_float, dp, dp, dp)
-    log = []
-
-    def res_cb(_, T16, expo, aff2, cut, out6):
-        T = np.array([T16[i] for i in range(16)]).reshape(4, 4)
-        r = t.calcRes(T, expo, np.array([aff2[0], aff2[1]]), cut)
-        log.append(("res", cut))
-        for i in range(6):
-            out6[i] = r[i]
-
-    def g_cb(_, expo, aff2, H64, b8):
-        H, b = t.calcG(expo, np.array([aff2[0], aff2[1]]))
-        for i in range(8):
-            b8[i] = b[i]
-            for j in range(8):
-                H64[8 * i + j] = H[i, j]
-    T0 = np.eye(4) if start == "identity" else np.array(c["refToNew"], np.float64) @ np.linalg.inv(
-        np.array([[1, 0, 0, 0.004], [0, 1, 0, -0.003], [0, 0, 1, 0.002], [0, 0, 0, 1.0]]))
-    T = np.ascontiguousarray(T0, np.float64).copy()
-    aff = np.array(c["ref_aff"], np.float64).copy()
-    out5 = np.zeros(5)
-    counts = (ctypes.c_int * 2)()
-    l.ref_lm_track_level0.restype = ctypes.c_int
-    ok = l.ref_lm_track_level0(None, RES(res_cb), G(g_cb), T.ctypes.data_as(dp), aff.ctypes.data_as(dp), ctypes.c_float(c["new_exposure"]),
-                               ctypes.c_float(c["ref_exposure"]), np.array(c["ref_aff"], np.float64).ctypes.data_as(dp),
-                               ctypes.c_float(cutoff), int(fix_a), int(fix_b), out5.ctypes.data_as(dp), counts)
+    g = np.load(golden_path("ref_lm.npz"))
+    k = lm_key(start, fix_a, fix_b, cutoff)
+    ok, counts, T, aff, out5 = int(g[k + "/ok"]), g[k + "/counts"], g[k + "/T"], g[k + "/aff"], g[k + "/out5"]
     assert ok == 1
+    c, t = lm_case()
+    T0 = lm_start(c, start)
     # the restatement: one pass, plus the reference's single REPEAT of the level when the cutoff had to be raised (:911-915)
     r = track_level0(t, T0, c["ref_aff"], c["new_exposure"], coarse_cutoff=cutoff, max_iterations=10, fix_a=fix_a, fix_b=fix_b)
     evals, passes = r["evaluations"], 1

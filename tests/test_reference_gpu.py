@@ -1,109 +1,70 @@
-"""Pins against the REAL reference, run on the same B200: oracle/_ref/ holds the reference's own dr_fusion class and
-tracker kernels compiled unmodified from /root/reference for sm_100a (oracle/ref_build.mk, built in the build
-container, shipped to the GPU box as a built .so; nothing from /root/reference is read at run time).
+"""Pins against the REAL reference: the reference's own dr_fusion class and tracker kernels, compiled unmodified for
+sm_100a (oracle/ref_build.mk) and run on a B200, produced the known answers in tests/golden/ref_gpu.npz
+(oracle/ref_golden.py); the same seeded inputs run here through the CUDA path and the CPU oracle.
 These tests are what lifts the TSDF / tracker oracles from "parity unpinned" to "pinned against the reference's
-CUDA code" (modulo the reference's documented races, SURVEY.md Appendix B)."""
-import ctypes
-import os
-
+CUDA code" (modulo the reference's documented races, SURVEY.md Appendix B).  Large reference outputs are stored as a
+fixed seeded sample (see oracle/ref_golden.py for which parts are complete)."""
 import numpy as np
 import pytest
 
-from oracle.cpu import TrackerOracle, TsdfOracle
-from tandem_b200 import CudaCoarseTracker, DrFusion, DrFusionOptions
-from tandem_b200.synthetic import RoomScene, circle_trajectory, tracker_case
+from oracle.ref_golden import (TRACKER_CASES, decode_depth, fusion_mesh_case, fusion_options, fusion_render_case, golden_path,
+                               tracker_oracle, tracker_ref_case)
+from oracle.cpu import TsdfOracle
+from tandem_b200 import CudaCoarseTracker, DrFusion
 
 pytestmark = pytest.mark.gpu
-REF_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-_fp = ctypes.POINTER(ctypes.c_float)
 
 
-def _ref_lib(name):
-    p = os.path.join(REF_DIR, name)
-    if not os.path.exists(p):
-        pytest.skip(f"{name} not built (oracle/ref_build.mk needs /root/reference)")
-    return ctypes.CDLL(p)
+@pytest.fixture(scope="module")
+def ref():
+    return np.load(golden_path("ref_gpu.npz"))
 
 
-def test_fusion_matches_reference_dr_fusion():
-    l = _ref_lib("libdr_fusion_ref.so")
-    l.ref_fusion_create.restype = ctypes.c_void_p
-    H, W = 120, 160
-    intr = dict(fx=80.0, fy=80.0, cx=79.5, cy=59.5)
-    opt = DrFusionOptions(height=H, width=W, num_buckets=200003, bucket_size=10, num_blocks=120000, **intr)
-    # world shifted by +2.56 m (32 blocks): the reference also integrates its FREE hash entries, all aliased to block (0,0,0)
-    # (Appendix B.2); keeping the origin far outside the map keeps that quirk out of the comparison.
-    off = np.array([2.56, 2.56, 2.56], np.float32)
-    scene = RoomScene(half=1.2, spheres=((0.5, 0.1, 0.4, 0.3), (-0.4, -0.2, 0.6, 0.25), (0.1, 0.4, -0.6, 0.3)))
-    poses = circle_trajectory(2, radius=0.3)
-    poses = [poses[0], poses[0].copy(), poses[1], poses[1].copy()]
-    poses[1][:3, 3] += np.float32(0.03)
-    poses[3][:3, 3] -= np.float32(0.02)
-    frames = [scene.render(p, H, W, **intr, noise_sigma=0.002, dropout=0.02, seed=k) for k, p in enumerate(poses)]
-    for p in poses:
-        p[:3, 3] += off
-    ref = ctypes.c_void_p(l.ref_fusion_create(ctypes.byref(opt)))
+def test_fusion_matches_reference_dr_fusion(ref):
+    opt = fusion_options()
+    H, W = opt.height, opt.width
+    poses, frames, render_poses = fusion_render_case()
     ours, orc = DrFusion(opt), TsdfOracle(opt)
-    try:
-        for k, (pose, (bgr, depth)) in enumerate(zip(poses, frames)):
-            b, d = np.ascontiguousarray(bgr), np.ascontiguousarray(depth)
-            l.ref_fusion_integrate(ref, ctypes.c_void_p(b.ctypes.data), d.ctypes.data_as(_fp), pose.ctypes.data_as(_fp))
-            ours.IntegrateScanAsync(bgr, depth, pose)
-            orc.integrate(bgr, depth, pose)
-            rp = poses[max(k - 1, 0)] if k % 2 else pose
-            rb = np.zeros((H, W, 3), np.uint8)
-            rd = np.zeros((H, W), np.float32)
-            l.ref_fusion_render(ref, rp.ctypes.data_as(_fp), ctypes.c_void_p(rb.ctypes.data), rd.ctypes.data_as(_fp), H * W)
-            ours.RenderAsync([rp])
-            (ob,), (od,) = ours.GetRenderResult()
-            cb, cd = orc.render(rp)
-            for name, xd, xb in (("cuda", od, ob), ("oracle", cd, cb)):
-                hit_r, hit_x = rd > 0, xd > 0
-                mism = float(np.mean(hit_r != hit_x))
-                both = hit_r & hit_x
-                err = np.abs(rd[both] - xd[both])
-                print(f"frame {k} {name} vs reference: hit mismatch {mism:.5f}, depth mean-abs {err.mean():.2e}, "
-                      f"max {err.max():.2e}, bit-equal {np.mean(rd == xd):.5f}, colour equal {np.mean(rb == xb):.5f}")
-                # the reference itself is FMA-contracted, uses a different 4x4 inverse and sphere-traces, so "same
-                # surface to a small fraction of a voxel" is the strongest statement available (voxel = 1e-2 m)
-                assert mism <= 3e-3
-                assert err.mean() <= 3e-4 and np.quantile(err, 0.99) <= 5e-3
-                assert np.mean(np.abs(rb[both].astype(int) - xb[both].astype(int)) <= 2) > 0.98
-    finally:
-        l.ref_fusion_destroy(ref)
+    for k, (pose, (bgr, depth), rp) in enumerate(zip(poses, frames, render_poses)):
+        ours.IntegrateScanAsync(bgr, depth, pose)
+        orc.integrate(bgr, depth, pose)
+        ours.RenderAsync([rp])
+        (ob,), (od,) = ours.GetRenderResult()
+        cb, cd = orc.render(rp)
+        rd = decode_depth(ref[f"render/{k}/depth_q"]).reshape(-1)
+        idx, rb = ref[f"render/{k}/idx"], ref[f"render/{k}/bgr"]      # colour: a seeded sample of the pixels
+        for name, xd, xb in (("cuda", od, ob), ("oracle", cd, cb)):
+            xd, xb = xd.reshape(-1), xb.reshape(-1, 3)[idx]
+            hit_r, hit_x = rd > 0, xd > 0
+            mism = float(np.mean(hit_r != hit_x))
+            both = hit_r & hit_x
+            err = np.abs(rd[both] - xd[both])
+            both_s = both[idx]
+            print(f"frame {k} {name} vs reference: hit mismatch {mism:.5f}, depth mean-abs {err.mean():.2e}, "
+                  f"max {err.max():.2e}, colour equal {np.mean(rb == xb):.5f} (on {idx.size} sampled pixels)")
+            # the reference itself is FMA-contracted, uses a different 4x4 inverse and sphere-traces, so "same
+            # surface to a small fraction of a voxel" is the strongest statement available (voxel = 1e-2 m)
+            assert mism <= 3e-3
+            assert err.mean() <= 3e-4 and np.quantile(err, 0.99) <= 5e-3
+            assert np.mean(np.abs(rb[both_s].astype(int) - xb[both_s].astype(int)) <= 2) > 0.98
 
 
-@pytest.mark.parametrize("size,step", [((120, 160), 1), ((480, 640), 1)])
-def test_tracker_matches_reference_kernels(size, step):
-    l = _ref_lib("libtracker_ref.so")
-    h, w = size
-    s = w / 640.0
-    c = tracker_case(H=h, W=w, fx=320.0 * s, fy=320.0 * s, cx=319.5 * s, cy=239.5 * s, step=step)
+@pytest.mark.parametrize("size,step", TRACKER_CASES)
+def test_tracker_matches_reference_kernels(ref, size, step):
+    c = tracker_ref_case(size, step)
     n = c["n"]
-    orc = TrackerOracle(w, h)
-    orc.setK(w, h, c["fx"], c["fy"], c["cx"], c["cy"])
-    orc.setReference(n, c["pc_u"], c["pc_v"], c["pc_idepth"], c["pc_color"], c["ref_exposure"], c["ref_aff"])
-    orc.setNew(c["dInew"])
+    orc = tracker_oracle(c)
     ro = orc.calcRes(c["refToNew"], c["new_exposure"], c["new_aff"], c["cutoffTH"])
     Ho, bo = orc.calcG(c["new_exposure"], c["new_aff"])
-    aff = orc._aff(c["new_exposure"], c["new_aff"])
-    T = np.ascontiguousarray(c["refToNew"], np.float32)
-    Ki = np.array([1.0 / c["fx"], 0, -c["cx"] / c["fx"], 0, 1.0 / c["fy"], -c["cy"] / c["fy"], 0, 0, 1], np.float32)
-    o7, o45 = np.zeros(7, np.float32), np.zeros(45, np.float32)
-    warped = np.zeros((7, n), np.float32)
-    f = ctypes.c_float
-    rc = l.ref_tracker_eval(w, h, f(c["fx"]), f(c["fy"]), f(c["cx"]), f(c["cy"]), T.ctypes.data_as(_fp), Ki.ctypes.data_as(_fp),
-                            f(aff[0]), f(aff[1]), f(c["ref_aff"][1]), f(9.0), f(c["cutoffTH"]), n,
-                            c["pc_u"].ctypes.data_as(_fp), c["pc_v"].ctypes.data_as(_fp), c["pc_idepth"].ctypes.data_as(_fp),
-                            c["pc_color"].ctypes.data_as(_fp), np.ascontiguousarray(c["dInew"]).ctypes.data_as(_fp),
-                            o7.ctypes.data_as(_fp), o45.ctypes.data_as(_fp), warped.ctypes.data_as(_fp))
-    assert rc == 0
+    key = f"tracker/{size[0]}x{size[1]}/{step}"
+    o7, o45 = ref[key + "/o7"], ref[key + "/o45"]
     # reference host post-processing (cuda_coarse_tracker.cpp:264-272, 335-355)
     rr = np.array([o7[0], o7[1], o7[4] / o7[6], 0, o7[5] / o7[6], o7[3] / o7[1]], np.float64)
     scale = np.array([1, 1, 1, .5, .5, .5, 10, 1000.0])
     tri = lambda r, q: min(r, q) * 9 + max(r, q) - min(r, q) * (min(r, q) + 1) // 2
     Hr = np.array([[o45[tri(r, q)] for q in range(8)] for r in range(8)], np.float64) / o7[2] * np.outer(scale, scale)
     br = np.array([o45[tri(r, 8)] for r in range(8)], np.float64) / o7[2] * scale
+    w, h = c["w"], c["h"]
     g = CudaCoarseTracker(w, h)
     g.init()
     g.setK(w, h, c["fx"], c["fy"], c["cx"], c["cy"])
@@ -120,61 +81,47 @@ def test_tracker_matches_reference_kernels(size, step):
         assert abs(r_[5] - rr[5]) <= 1e-4
         assert rel(H_, Hr) < 2e-3 and rel(b_, br) < 2e-3   # reference sums 3e5 fp32 terms with float atomics
     wo = orc.warped
-    same = (warped[6] != 0) == (wo[6] != 0)
+    valid = np.unpackbits(ref[key + "/valid"], count=n).astype(bool)
+    same = valid == (wo[6] != 0)
     assert same.mean() > 0.9999
-    m = (warped[6] != 0) & (wo[6] != 0)
-    assert np.quantile(np.abs(warped[5][m] - wo[5][m]), 0.999) < 5e-3 and np.max(np.abs(warped[5][m] - wo[5][m])) < 5e-2
+    idx = ref[key + "/idx"]                 # residuals: a seeded sample of the points
+    m = valid[idx] & (wo[6][idx] != 0)
+    d = np.abs(ref[key + "/residual"][m] - wo[5][idx][m])
+    assert np.quantile(d, 0.999) < 5e-3 and np.max(d) < 5e-2
 
 
-def test_mesh_matches_reference_marching_cubes():
+def test_mesh_matches_reference_marching_cubes(ref):
     """DrFusion::GetMesh of the reference (brute-force ExtractMeshKernel, mesh_extractor.cu:244-265) vs ours and vs the
     oracle on volumes fused from the same scans.  The volumes themselves differ in the last bits (FMA contraction, 4x4
     inverse, allocation races - see the render test above), so the meshes are compared as surfaces: triangle counts
-    within 2 %, and every vertex of one mesh has a vertex of the other within a small fraction of a voxel."""
+    within 2 %, inside a crop cube (where the reference mesh is stored in full) every vertex of ours has a reference vertex
+    within a small fraction of a voxel, and so has every sampled vertex of the reference mesh one of ours."""
     from scipy.spatial import cKDTree
-    l = _ref_lib("libdr_fusion_ref.so")
-    l.ref_fusion_create.restype = ctypes.c_void_p
-    l.ref_fusion_get_mesh.restype = ctypes.c_longlong
-    H, W = 120, 160
-    intr = dict(fx=80.0, fy=80.0, cx=79.5, cy=59.5)
-    opt = DrFusionOptions(height=H, width=W, num_buckets=200003, bucket_size=10, num_blocks=120000, **intr)
-    off = np.array([2.56, 2.56, 2.56], np.float32)
-    scene = RoomScene(half=1.2, spheres=((0.5, 0.1, 0.4, 0.3), (-0.4, -0.2, 0.6, 0.25), (0.1, 0.4, -0.6, 0.3)))
-    poses = circle_trajectory(3, radius=0.3)
-    frames = [scene.render(p, H, W, **intr, noise_sigma=0.002, dropout=0.02, seed=k) for k, p in enumerate(poses)]
-    for p in poses:
-        p[:3, 3] += off
-    ref = ctypes.c_void_p(l.ref_fusion_create(ctypes.byref(opt)))
+    opt = fusion_options()
+    poses, frames, lo, up = fusion_mesh_case()
     ours, orc = DrFusion(opt), TsdfOracle(opt)
-    try:
-        for pose, (bgr, depth) in zip(poses, frames):
-            b, d = np.ascontiguousarray(bgr), np.ascontiguousarray(depth)
-            l.ref_fusion_integrate(ref, ctypes.c_void_p(b.ctypes.data), d.ctypes.data_as(_fp), pose.ctypes.data_as(_fp))
-            rb = np.zeros((H, W, 3), np.uint8); rd = np.zeros((H, W), np.float32)
-            l.ref_fusion_render(ref, pose.ctypes.data_as(_fp), ctypes.c_void_p(rb.ctypes.data), rd.ctypes.data_as(_fp), H * W)
-            ours.IntegrateScanAsync(bgr, depth, pose)
-            ours.RenderAsync([pose]); ours.GetRenderResult()
-            orc.integrate(bgr, depth, pose)
-        lo = (off - np.float32(1.28)).astype(np.float32)
-        up = (off + np.float32(1.28)).astype(np.float32)
-        cap = 3 * 2000000
-        rv = np.zeros((cap, 3), np.float32); rc = np.zeros((cap, 3), np.float32)
-        n = l.ref_fusion_get_mesh(ref, lo.ctypes.data_as(_fp), up.ctypes.data_as(_fp), rv.ctypes.data_as(_fp), rc.ctypes.data_as(_fp),
-                                  ctypes.c_longlong(cap))
-        assert 0 < n <= cap
-        rv, rc = rv[:n], rc[:n]
-        gv, gc = ours.GetMesh(lo, up)
-        ov, oc = orc.extract_mesh(lo, up)
-        tree = cKDTree(rv)
-        for name, xv, xc in (("cuda", gv, gc), ("oracle", ov, oc)):
-            dist, idx = tree.query(xv)
-            back, _ = cKDTree(xv).query(rv)
-            exact = float(np.mean(dist == 0))
-            print(f"{name} vs reference mesh: {len(xv) // 3} vs {n // 3} triangles, vertex NN distance median {np.median(dist):.2e} "
-                  f"p99 {np.quantile(dist, 0.99):.2e} (reverse p99 {np.quantile(back, 0.99):.2e}), coincident vertices {exact:.4f}, "
-                  f"colour max diff at NN (median) {np.median(np.abs(xc - rc[idx]).max(1)):.3f}")
-            assert abs(len(xv) - n) <= 0.02 * n
-            assert np.median(dist) <= 1e-4 and np.quantile(dist, 0.99) <= 5e-3 and np.quantile(back, 0.99) <= 5e-3
-            assert np.median(np.abs(xc - rc[idx]).max(1)) <= 2.5 / 255
-    finally:
-        l.ref_fusion_destroy(ref)
+    for pose, (bgr, depth) in zip(poses, frames):
+        ours.IntegrateScanAsync(bgr, depth, pose)
+        ours.RenderAsync([pose]); ours.GetRenderResult()
+        orc.integrate(bgr, depth, pose)
+    n = int(ref["mesh/n"])
+    sv = ref["mesh/sample_vert"]
+    clo, cup = ref["mesh/crop_lo"], ref["mesh/crop_up"]
+    cv, cc = ref["mesh/crop_vert"], ref["mesh/crop_color"].astype(np.float32)
+    gv, gc = ours.GetMesh(lo, up)
+    ov, oc = orc.extract_mesh(lo, up)
+    tree = cKDTree(cv)
+    margin = np.float32(0.01)           # one voxel: the nearest reference vertex of a vertex this far inside is in the crop
+    for name, xv, xc in (("cuda", gv, gc), ("oracle", ov, oc)):
+        inner = np.all((xv >= clo + margin) & (xv <= cup - margin), axis=1)
+        assert inner.sum() > 100, (name, int(inner.sum()))
+        dist, idx = tree.query(xv[inner])
+        back, _ = cKDTree(xv).query(sv)
+        exact = float(np.mean(dist == 0))
+        print(f"{name} vs reference mesh: {len(xv) // 3} vs {n // 3} triangles, vertex NN distance median {np.median(dist):.2e} "
+              f"p99 {np.quantile(dist, 0.99):.2e} ({int(inner.sum())} vertices in the crop; reverse p99 {np.quantile(back, 0.99):.2e} "
+              f"over {len(sv)} sampled reference vertices), coincident vertices {exact:.4f}, "
+              f"colour max diff at NN (median) {np.median(np.abs(xc[inner] - cc[idx]).max(1)):.3f}")
+        assert abs(len(xv) - n) <= 0.02 * n
+        assert np.median(dist) <= 1e-4 and np.quantile(dist, 0.99) <= 5e-3 and np.quantile(back, 0.99) <= 5e-3
+        assert np.median(np.abs(xc[inner] - cc[idx]).max(1)) <= 2.5 / 255
